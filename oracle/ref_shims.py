@@ -1,9 +1,8 @@
 """ORACLE tooling: import the reference's OWN Python modules (read-only, from /root/reference) in a container that
 lacks diffusers / accelerate / xformers / omegaconf / IPython, by installing minimal stub modules in sys.modules.
 
-Only used (a) by tests/golden/make_golden.py to generate the committed golden vectors and (b) by
-tests/test_oracle_vs_reference.py, which is skipped wherever /root/reference does not exist (e.g. the GPU box).
-Nothing under /root/reference is copied; the modules are executed in place.
+Only used by tests/golden/make_golden.py to generate the committed golden vectors, which the tests compare against.
+Nothing of the reference is copied; the modules are executed in place.
 """
 import importlib.machinery
 import importlib.util

@@ -1,6 +1,6 @@
 """Generate tests/golden/reference_golden.pt by executing the REFERENCE's own Python (read-only, in place, under the
-import shims of oracle/ref_shims.py) on seeded synthetic inputs.  Run in the build container, where /root/reference
-exists:   python tests/golden/make_golden.py
+import shims of oracle/ref_shims.py) on seeded synthetic inputs.  Run where a checkout of the reference exists (its
+directory in MOS_REFERENCE_ROOT):   python tests/golden/make_golden.py   (--crosscheck: tests/golden/reference_crosscheck.pt)
 The reference ships no tests or golden vectors (SURVEY.md §4); these fixtures are what pins the oracle.
 Third-party diffusers is absent, so the skeleton the reference code runs on is oracle/unet.py (see its header).
 """
@@ -17,6 +17,7 @@ from oracle import ref_shims  # noqa: E402
 from oracle import unet as ou  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'reference_golden.pt')
+CROSS = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'reference_crosscheck.pt')
 
 
 def gen(seed):
@@ -84,8 +85,56 @@ def golden_attn_reg():
     return out
 
 
+def crosscheck():
+    """What the reference's own modules return on the cases of tests/test_oracle_vs_reference.py and of the mirror check in
+    tests/test_checkpoint_formats.py, and the parsed options of a shipped training yml -> reference_crosscheck.pt."""
+    import yaml
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import test_checkpoint_formats as tc
+    import test_oracle_vs_reference as tv
+    ed = ref_shims.load_reference_module('mixofshow/models/edlora.py')
+    pe = ref_shims.load_reference_module('mixofshow/pipelines/pipeline_edlora.py')
+    gf = ref_shims.load_reference_module('gradient_fusion.py')
+    cv = ref_shims.load_reference_module('mixofshow/utils/convert_edlora_to_diffusers.py')
+    G = {}
+
+    unet, lora, x, ehs = tv.installer_case()
+    ed.revise_edlora_unet_attention_forward(unet)
+    mods = dict(unet.named_modules())
+    keep = []
+    for k in lora:
+        if k.endswith('.lora_down.weight'):
+            n = k[:-len('.lora_down.weight')]
+            layer = ed.LoRALinearLayer(n, mods[n], rank=4, alpha=tv.LORA_ALPHA)
+            layer.lora_down.weight.data = lora[k].clone()
+            layer.lora_up.weight.data = lora[n + '.lora_up.weight'].clone()
+            keep.append(layer)
+    with torch.no_grad():
+        G['installer'] = dict(out=unet(x, torch.tensor([500, 500]), ehs).sample, n_lora=len(keep))
+
+    G['bind_concept_prompt'] = pe.bind_concept_prompt(tv.BIND_PROMPTS, tv.BIND_CFG)
+    K, V, W0 = tv.quasi_newton_case()
+    G['quasi_newton'] = dict(K=K, V=V, W0=W0, W=gf.update_quasi_newton(K, V, W0.clone(), tv.QN_ITERS, 'cpu').detach())
+
+    sds, ckpt = tc.mirror_case()
+    merge = {}
+    for model_type, sd in sds.items():
+        merged = cv.merge_lora_into_weight(sd, ckpt[model_type], model_type=model_type, alpha=tc.MERGE_ALPHA)
+        merge[model_type] = tc.merge_samples(sd, merged)
+    G['convert'] = dict(merge=merge, load_new_concept=tc.load_concept(cv.load_new_concept, ckpt['new_concept_embedding']))
+
+    with open(os.path.join(ref_shims.REFERENCE_ROOT, 'options/train/EDLoRA/real/8101_EDLoRA_potter_Cmix_B4_Repeat500.yml')) as f:
+        opt = yaml.safe_load(f)
+    G['train_options'] = dict(models=opt['models'], train=dict(emb_norm_threshold=opt['train']['emb_norm_threshold']))
+    torch.save(G, CROSS)
+    print('wrote', CROSS, os.path.getsize(CROSS) / 1e6, 'MB')
+
+
 def main():
     assert ref_shims.reference_available(), 'needs /root/reference'
+    if '--crosscheck' in sys.argv:
+        crosscheck()
+        return
     if '--only-attn-reg' in sys.argv:
         G = torch.load(OUT, weights_only=False)
         G['attn_reg'] = golden_attn_reg()

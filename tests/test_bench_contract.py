@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -40,7 +42,6 @@ def test_reference_arm_nonzero_rank_is_silent():
 def test_product_arm_fails_loudly_without_cuda():
     import torch
     if torch.cuda.is_available():
-        import pytest
         pytest.skip('a GPU is present')
     r = _run(['--tiny', '--steps', '1', '--warmup', '1'])
     assert r.returncode != 0 and 'needs a GPU' in (r.stderr + r.stdout)
@@ -63,3 +64,34 @@ def test_product_code_never_imports_the_oracle():
         head = src[:m.start()]
         last_def = head.rfind('\ndef ')
         assert src[last_def + 1:].startswith(allowed), 'bench.py imports oracle outside the CPU-baseline functions'
+
+
+def test_dump_outputs_writes_float32_within_budget(tmp_path, monkeypatch):
+    """An array over its share of the budget is replaced by the same seeded sample of its elements every time."""
+    import numpy as np
+    import torch
+
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 4096)
+    big = torch.arange(5000, dtype=torch.float64).view(50, 100)
+    small = torch.ones(2, 3, dtype=torch.float16)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), {'big': big, 'small': small})
+    a, b = np.load(tmp_path / 'a' / 'big.npy'), np.load(tmp_path / 'b' / 'big.npy')
+    assert a.dtype == np.float32 and a.shape == (512,) and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0) and np.all(np.isin(a, big.numpy()))
+    s = np.load(tmp_path / 'a' / 'small.npy')
+    assert s.dtype == np.float32 and s.shape == (2, 3) and np.all(s == 1)
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_its_outputs(cuda, tmp_path):
+    import numpy as np
+    r = _run(['--tiny', '--steps', '2', '--warmup', '1', '--no-train', '--no-cpu-baseline', '--dump-outputs', str(tmp_path)])
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])['steps'] == 2
+    shapes = {'latents': (1, 4, 64, 64), 'eps': (2, 4, 64, 64), 'e2e_latents': (1, 4, 64, 64)}
+    assert sorted(os.listdir(tmp_path)) == sorted(n + '.npy' for n in shapes)
+    for n, shape in shapes.items():
+        a = np.load(tmp_path / (n + '.npy'))
+        assert a.dtype == np.float32 and a.shape == shape and np.isfinite(a).all(), n

@@ -1,13 +1,16 @@
 """On-disk / checkpoint plumbing (SURVEY.md 8f rank 3), CPU only: the ED-LoRA delta checkpoint layout
 (trainer_edlora.py:358-378, train_edlora.py:168-171) loaded through this repo's `convert_edlora_to_diffusers` mirror into
-this repo's containers, cross-checked live against the reference's own file where /root/reference exists."""
+this repo's containers, cross-checked against what the reference's own file returned (tests/golden/reference_crosscheck.pt)."""
 import io
+import os
 
 import pytest
 import torch
 
-from oracle import inject, ref_shims
+from oracle import inject
 from oracle import unet as ou
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_crosscheck.pt')
 
 
 class FakeTokenizer:
@@ -125,29 +128,52 @@ def test_clip_container_embedding_surface(monkeypatch):
         te.load_state_dict({'nope': torch.zeros(1)})
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason='reference checkout not present')
-def test_mirror_matches_reference_file_live():
-    from types import SimpleNamespace
-    from mixofshow.utils import convert_edlora_to_diffusers as mine
-    ref = ref_shims.load_reference_module('mixofshow/utils/convert_edlora_to_diffusers.py')
+MERGE_ALPHA = 0.7
+
+
+def mirror_case():
+    """Tiny UNet (seed 0) and one-layer CLIP text encoder state dicts, and a seeded delta checkpoint (seed 5)."""
     unet = ou.build_unet(0, ou.TINY)
     clip, clip_sd = _clip_sd()
-    ckpt = _delta(unet, clip, seed=5)['params']
-    for model_type, sd in (('unet', unet.state_dict()), ('text_encoder', clip_sd)):
-        a = ref.merge_lora_into_weight(sd, ckpt[model_type], model_type=model_type, alpha=0.7)
-        b = mine.merge_lora_into_weight(sd, ckpt[model_type], model_type=model_type, alpha=0.7)
-        assert a.keys() == b.keys()
-        assert all(torch.equal(a[k], b[k]) for k in a)
-        changed = sum(not torch.equal(a[k], sd[k]) for k in a)
-        assert changed == len(ckpt[model_type]) // 2
-    # load_new_concept on the reference's kind of objects (transformers CLIPTextModel + tokenizer stand-in)
+    return {'unet': unet.state_dict(), 'text_encoder': clip_sd}, _delta(unet, clip, seed=5)['params']
+
+
+def merge_samples(sd, merged, n=64):
+    """The keys of a merged state dict and, for every tensor the merge changed, a fixed seeded sample of its elements."""
+    g = torch.Generator().manual_seed(0)
+    samples = {}
+    for k in sorted(k for k in merged if not torch.equal(merged[k], sd[k])):
+        idx = torch.randint(0, merged[k].numel(), (n,), generator=g)
+        samples[k] = (idx, merged[k].flatten()[idx].clone())
+    return sorted(merged), samples
+
+
+def load_concept(load_new_concept, embeddings):
+    """load_new_concept on the reference's kind of objects (transformers CLIPTextModel + tokenizer stand-in)."""
+    from types import SimpleNamespace
     from transformers import CLIPTextConfig, CLIPTextModel
-    outs = []
-    for fn in (ref.load_new_concept, mine.load_new_concept):
-        torch.manual_seed(0)
-        m = CLIPTextModel(CLIPTextConfig(vocab_size=300, hidden_size=768, intermediate_size=3072, num_hidden_layers=1,
-                                         num_attention_heads=12, max_position_embeddings=77))
-        pipe = SimpleNamespace(tokenizer=FakeTokenizer(300), text_encoder=m)
-        pipe, cfg = fn(pipe, ckpt['new_concept_embedding'], True)
-        outs.append((cfg, m.get_input_embeddings().weight.data[300:].clone()))
-    assert outs[0][0] == outs[1][0] and torch.equal(outs[0][1], outs[1][1])
+    torch.manual_seed(0)
+    m = CLIPTextModel(CLIPTextConfig(vocab_size=300, hidden_size=768, intermediate_size=3072, num_hidden_layers=1,
+                                     num_attention_heads=12, max_position_embeddings=77))
+    pipe = SimpleNamespace(tokenizer=FakeTokenizer(300), text_encoder=m)
+    pipe, cfg = load_new_concept(pipe, embeddings, True)
+    return cfg, m.get_input_embeddings().weight.data[300:].clone()
+
+
+def test_mirror_matches_reference_file_live():
+    """The mirror's merge and concept load reproduce what the reference's convert_edlora_to_diffusers.py returned on the same
+    case (stored by tests/golden/make_golden.py --crosscheck)."""
+    from mixofshow.utils import convert_edlora_to_diffusers as mine
+    gold = torch.load(GOLD, weights_only=False)['convert']
+    sds, ckpt = mirror_case()
+    for model_type, sd in sds.items():
+        merged = mine.merge_lora_into_weight(sd, ckpt[model_type], model_type=model_type, alpha=MERGE_ALPHA)
+        keys, samples = merge_samples(sd, merged)
+        gkeys, gsamples = gold['merge'][model_type]
+        assert keys == gkeys and samples.keys() == gsamples.keys()
+        assert len(samples) == len(ckpt[model_type]) // 2
+        for k, (idx, vals) in samples.items():
+            assert torch.equal(idx, gsamples[k][0])
+            assert torch.allclose(vals, gsamples[k][1], rtol=1e-6, atol=1e-8), k
+    cfg, rows = load_concept(mine.load_new_concept, ckpt['new_concept_embedding'])
+    assert cfg == gold['load_new_concept'][0] and torch.equal(rows, gold['load_new_concept'][1])

@@ -184,12 +184,10 @@ def test_regional_script_prepare_text_matches_reference_golden():
 
 def test_latent_dataset_and_yml_options(tmp_path):
     """`train_edlora.py -opt <yml>` host side: LatentDataset (replace_mapping, dataset_enlarge_ratio, per-rank sharding of one
-    shared permutation, drop_last) and the shipped reference yml parsing (`!!float` tags, models block = EDLoRATrainer
+    shared permutation, drop_last) and the options of a shipped reference yml (`!!float` values, models block = EDLoRATrainer
     keyword arguments)."""
     import inspect
     import os
-
-    import yaml
 
     import train_edlora as te
     from mixofshow.pipelines.trainer_edlora import EDLoRATrainer
@@ -206,9 +204,9 @@ def test_latent_dataset_and_yml_options(tmp_path):
         assert b0['images'].shape == (2, 4, 2, 2) and len(b0['prompts']) == 2 and b0['masks'].shape == (2, 1, 2, 2)
         seen += [int(x[0, 0, 0]) // 16 for x in list(b0['images']) + list(b1['images'])]
     assert len(seen) == 28 and max(seen.count(i) for i in range(6)) <= 5
-    ref_yml = '/root/reference/options/train/EDLoRA/real/8101_EDLoRA_potter_Cmix_B4_Repeat500.yml'
-    if os.path.exists(ref_yml):
-        opt = yaml.safe_load(open(ref_yml))
-        assert opt['models']['finetune_cfg']['text_embedding']['lr'] == 1e-3 and opt['train']['emb_norm_threshold'] == 0.55
-        params = inspect.signature(EDLoRATrainer.__init__).parameters
-        assert all(k in params for k in opt['models']), 'EDLoRATrainer(**opt["models"]) must accept every key of the yml'
+    # the parsed options of the reference's 8101_EDLoRA_potter_Cmix_B4_Repeat500.yml (tests/golden/make_golden.py --crosscheck)
+    gold = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_crosscheck.pt')
+    opt = torch.load(gold, weights_only=False)['train_options']
+    assert opt['models']['finetune_cfg']['text_embedding']['lr'] == 1e-3 and opt['train']['emb_norm_threshold'] == 0.55
+    params = inspect.signature(EDLoRATrainer.__init__).parameters
+    assert all(k in params for k in opt['models']), 'EDLoRATrainer(**opt["models"]) must accept every key of the yml'
