@@ -40,6 +40,7 @@ const char* mos_last_error(void);
 enum { MOS_DT_BF16 = 0, MOS_DT_F16 = 1 };   /* 16-bit storage type of activations (`act_dtype` arguments) */
 enum { MOS_OUT_BF16 = 0 /* 16-bit rows of type a_dtype */, MOS_OUT_HEADS = 1, MOS_OUT_F32 = 2 };
 enum { MOS_SEG_ROWS = 0 /* [b,h,row,dpad] (Q, K) */, MOS_SEG_TRANSPOSED = 1 /* [b,h,d,row] (V^T) */ };
+enum { MOS_ACT_NONE = 0, MOS_ACT_RELU = 1 };   /* epilogue activation (`act`) */
 
 typedef struct mos_gemm_args {
   const void* A;          /* bf16 [M, lda]; conv: NHWC activation [B, H, Wd, C] */
@@ -86,6 +87,8 @@ typedef struct mos_gemm_args {
   const void* prefetch_ptr;    /* optional: [prefetch_bytes] of STATIC device data (normally the next layer's weights) that the
                                 * launch pulls into L2 with cp.async.bulk.prefetch.L2 while it runs; semantically a no-op */
   int64_t prefetch_bytes;
+  int32_t act;            /* MOS_ACT_*: out = act(acc + bias) (+ residual), in fp32 before rounding (T2I-Adapter resnet
+                           * block1).  Needs 16-bit row output without split-K / geglu / LoRA. */
 } mos_gemm_args;
 
 int mos_gemm_bf16(const mos_gemm_args* args, void* stream);
@@ -160,6 +163,17 @@ int mos_im2col_s2(const void* x, int64_t ldx, int32_t B, int32_t H, int32_t W, i
 /* x[m, :C] += r[m, :C] (T2I-Adapter residuals, pipeline_regionally_t2iadapter.py:565). */
 int mos_add_rows(void* x, int64_t ldx, const void* r, int64_t ldr, int64_t M, int32_t C, int32_t act_dtype,
                  void* stream);
+
+/* ---- T2I-Adapter (diffusers T2IAdapter, adapter_type 'full_adapter', run once per condition image at
+ * pipeline_regionally_t2iadapter.py:474-482).  Its 3x3 / 1x1 convolutions reuse mos_gemm_bf16 (conv / plain, MOS_ACT_RELU). */
+/* PixelUnshuffle(r): fp32 NCHW [B, C, H, W] -> 16-bit NHWC rows [B*(H/r)*(W/r), ldy], column c*r*r + i*r + j =
+ * x[b, c, ho*r + i, wo*r + j] (torch's channel order).  H, W multiples of r; C*r*r a multiple of 8. */
+int mos_pixel_unshuffle(const float* x, int32_t B, int32_t C, int32_t H, int32_t W, int32_t r, void* y, int64_t ldy,
+                        int32_t act_dtype, void* stream);
+/* AvgPool2d(2, 2, ceil_mode=True): 16-bit NHWC [B, H, W, ldx] -> [B, ceil(H/2), ceil(W/2), ldy]; fp32 sum divided by the
+ * number of taps inside the input (odd H / W: the last row / column averages 2 or 1 taps). */
+int mos_avgpool2x2(const void* x, int64_t ldx, int32_t B, int32_t H, int32_t W, int32_t C, void* y, int64_t ldy,
+                   int32_t act_dtype, void* stream);
 
 /* ---- CLIP text encoder (SURVEY.md 8f rank 1; transformers CLIPTextModel called at pipeline_edlora.py:133-145,
  * trainer_edlora.py:220-234, gradient_fusion.py:182-199).  The linears and LayerNorms reuse mos_gemm_bf16 / mos_layernorm_fwd. */

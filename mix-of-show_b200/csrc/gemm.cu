@@ -73,6 +73,7 @@ struct GemmDev {
   int stg_alias;       // the epilogue staging tile overlays pipeline stage 0.. (launches with <= 1 work item per CTA)
   const uint8_t* pf;   // optional: bytes to pull into L2 for a LATER launch (the next layer's weights), see mos_gemm_args
   long long pf_bytes;
+  int act;             // MOS_ACT_*: applied to acc + bias (+ LoRA) before the residual
 };
 
 template <bool F16>
@@ -539,6 +540,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 o[j] += tt[0] * u.x + tt[1] * u.y + tt[2] * u.z + tt[3] * u.w;
               }
             }
+            if (p.act == MOS_ACT_RELU) {
+#pragma unroll
+              for (int j = 0; j < 16; ++j) o[j] = fmaxf(o[j], 0.f);
+            }
             if (p.out_mode == MOS_OUT_BF16) {
               if (p.residual) {
                 const uint4 r0 = *reinterpret_cast<const uint4*>(srow + nl * 2);
@@ -787,6 +792,10 @@ extern "C" int mos_gemm_bf16(const mos_gemm_args* a, void* stream_) {
   const bool f16 = a->a_dtype == MOS_DT_F16;
   const int splits = a->splits > 0 ? a->splits : 1;
   const bool lora = a->lora_down != nullptr;
+  MOS_CHECK_ARG(a->act == MOS_ACT_NONE || a->act == MOS_ACT_RELU, "mos_gemm_bf16: act=%d is not a MOS_ACT_* value", a->act);
+  if (a->act != MOS_ACT_NONE)
+    MOS_CHECK_ARG(splits == 1 && !lora && !a->geglu && a->out_mode == MOS_OUT_BF16,
+                  "mos_gemm_bf16: act needs 16-bit row output without split-K / geglu / LoRA / head-split / fp32 output");
   if (splits > 1) {
     MOS_CHECK_ARG(a->partial != nullptr, "mos_gemm_bf16: split-K needs a partial workspace");
     if (a->tile_counters != nullptr)
@@ -953,6 +962,7 @@ extern "C" int mos_gemm_bf16(const mos_gemm_args* a, void* stream_) {
   p.w_static = a->w_static;
   p.pf = nullptr;
   p.pf_bytes = 0;
+  p.act = a->act;
   if (a->prefetch_ptr != nullptr && a->prefetch_bytes >= 16) {
     MOS_CHECK_ARG(is_aligned(a->prefetch_ptr, 16), "mos_gemm_bf16: prefetch_ptr must be 16-byte aligned");
     p.pf = reinterpret_cast<const uint8_t*>(a->prefetch_ptr);

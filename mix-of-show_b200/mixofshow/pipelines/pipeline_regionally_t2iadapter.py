@@ -4,13 +4,15 @@
 The region-masked cross-attention (reference :32-86) runs as: one flash cross-attention per region with the region's
 own K/V (tcgen05), then `mos_region_combine` (global outside the boxes, mean of covering regions inside).  Box indices
 are computed on the host in Python float64 exactly as the reference does (`math.ceil` / `math.floor`), so they are
-bit-exact.  The T2I-Adapter networks themselves are out of scope (SURVEY.md §2.1 row 6): pass their four feature
-maps as `adapter_state` (or torch adapter modules as `keypose_adapter` / `sketch_adapter` attributes).
+bit-exact.  Condition images (`*_adapter_input`: PIL images or tensors) are preprocessed as diffusers does and run
+through the `keypose_adapter` / `sketch_adapter` attributes (mixofshow.models.adapter_b200.T2IAdapter on the B200);
+pre-computed feature maps can be passed as `*_adapter_state` instead.
 """
 import ast
 import math
 from types import SimpleNamespace
 
+import numpy as np
 import torch
 
 from mixofshow.pipelines.pipeline_edlora import bind_concept_prompt
@@ -87,6 +89,22 @@ def _spatial_weight(feat, base_weight, region_weight_str, height, width):
     return wmap * feat
 
 
+def _preprocess_adapter_image(image, height, width):
+    """diffusers' `_preprocess_adapter_image` (reference :413-423): a PIL image or a list of them -> LANCZOS resize to
+    (width, height) -> fp32 NCHW in [0, 1] (a grayscale image gets one channel); tensors pass through untouched."""
+    import PIL.Image
+    if isinstance(image, torch.Tensor):
+        return image
+    if isinstance(image, PIL.Image.Image):
+        image = [image]
+    if not (isinstance(image, (list, tuple)) and image and all(isinstance(i, PIL.Image.Image) for i in image)):
+        raise TypeError(f'adapter input must be a PIL image, a list of PIL images or a tensor, got {type(image)}')
+    arrs = [np.array(i.resize((width, height), resample=PIL.Image.LANCZOS)) for i in image]
+    arrs = [a[None, ..., None] if a.ndim == 2 else a[None] for a in arrs]
+    x = np.concatenate(arrs, axis=0).astype(np.float32) / 255.0
+    return torch.from_numpy(x.transpose(0, 3, 1, 2).copy())
+
+
 class RegionallyT2IAdapterPipeline:
     def __init__(self, vae=None, text_encoder=None, tokenizer=None, unet=None, scheduler=None, safety_checker=None,
                  feature_extractor=None, requires_safety_checker: bool = False):
@@ -143,6 +161,29 @@ class RegionallyT2IAdapterPipeline:
                 region_list[idx] = (torch.cat([rn, re_]), pos)
         return prompt_embeds, region_list
 
+    def _run_adapter(self, adapter, kind, adapter_input, height, width, latent_hw):
+        """reference :413-423 + :474-482: preprocess the condition and run the adapter once."""
+        if adapter is None:
+            raise ValueError(f'{kind}_adapter_input given but pipe.{kind}_adapter is not set')
+        x = _preprocess_adapter_image(adapter_input, height, width).to(self.device, adapter.dtype)
+        state = adapter(x)
+        if tuple(state[0].shape[-2:]) != tuple(latent_hw):
+            raise ValueError(f'{kind} adapter features are {tuple(state[0].shape[-2:])}, the latents {tuple(latent_hw)}: '
+                             'the adapter downscale factor must equal the VAE scale factor')
+        return state
+
+    @torch.no_grad()
+    def decode_latents(self, latents, output_type='pil'):
+        """latents -> images through the VAE: a list of PIL images, or an NHWC numpy array for output_type='np'."""
+        if self.vae is None:
+            raise ValueError("no VAE supplied: use output_type='latent'")
+        image = self.vae.decode(latents / 0.18215).sample
+        image = (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).float().numpy()
+        if output_type == 'pil':
+            from mixofshow.pipelines.pipeline_edlora import numpy_to_pil
+            image = numpy_to_pil(image)
+        return image
+
     @torch.no_grad()
     def __call__(self, prompt=None, keypose_adapter_input=None, keypose_adaptor_weight=1.0,
                  region_keypose_adaptor_weight='', sketch_adapter_input=None, sketch_adaptor_weight=1.0,
@@ -170,9 +211,11 @@ class RegionallyT2IAdapterPipeline:
         latents = (latents.to(device, torch.float32) * self.scheduler.init_noise_sigma).contiguous()
 
         if keypose_adapter_state is None and keypose_adapter_input is not None:
-            keypose_adapter_state = self.keypose_adapter(keypose_adapter_input)
+            keypose_adapter_state = self._run_adapter(self.keypose_adapter, 'keypose', keypose_adapter_input, height, width,
+                                                      (h, w))
         if sketch_adapter_state is None and sketch_adapter_input is not None:
-            sketch_adapter_state = self.sketch_adapter(sketch_adapter_input)
+            sketch_adapter_state = self._run_adapter(self.sketch_adapter, 'sketch', sketch_adapter_input, height, width,
+                                                     (h, w))
         adapter_state = None
         if keypose_adapter_state is not None or sketch_adapter_state is not None:
             n = len(keypose_adapter_state) if keypose_adapter_state is not None else len(sketch_adapter_state)
@@ -204,16 +247,7 @@ class RegionallyT2IAdapterPipeline:
                                t_next=t_next)
             if callback is not None and i % callback_steps == 0:
                 callback(i, t, latents)
-        if output_type == 'latent':
-            image = latents
-        else:
-            if self.vae is None:
-                raise ValueError("no VAE supplied: use output_type='latent'")
-            image = self.vae.decode(latents / 0.18215).sample
-            image = (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).float().numpy()
-            if output_type == 'pil':
-                from mixofshow.pipelines.pipeline_edlora import numpy_to_pil
-                image = numpy_to_pil(image)
+        image = latents if output_type == 'latent' else self.decode_latents(latents, output_type)
         if not return_dict:
             return (image, None)
         return SimpleNamespace(images=image, nsfw_content_detected=None)

@@ -5,6 +5,8 @@
         <dir>/unet/config.json + diffusion_pytorch_model.safetensors (or .bin)
         <dir>/text_encoder/config.json + model.safetensors (or pytorch_model.bin)
   * `<dir>/new_concept_cfg.json` (`gradient_fusion.py:812-813`).
+  * a T2I-Adapter directory (`config.json` + `diffusion_pytorch_model.safetensors`, what
+    `T2IAdapter.from_pretrained` reads at `regionally_controlable_sampling.py:62-63`).
 
 `load_unet` / `load_text_encoder` build this repo's B200 containers from such a directory; `save_combined_model` writes
 one.  diffusers itself is not a dependency: the UNet `config.json` keys are the SD1.5 ones (diffusers 0.19.3), and any
@@ -170,6 +172,36 @@ def save_vae(vae, model_dir, subfolder='vae'):
     with open(os.path.join(folder, 'config.json'), 'w') as f:
         json.dump(cfg, f, indent=2, sort_keys=True)
     _write_weights(folder, VAE_WEIGHTS[0], vae.state_dict())
+
+
+ADAPTER_WEIGHTS = ('diffusion_pytorch_model.safetensors', 'diffusion_pytorch_model.bin')
+
+
+def load_t2i_adapter(model_dir, device='cuda'):
+    """diffusers-layout T2IAdapter directory (config.json + weights, e.g. a local copy of TencentARC/t2iadapter_openpose_sd14v1)
+    -> mixofshow.models.adapter_b200.T2IAdapter.  The config is validated by the T2IAdapter constructor."""
+    from mixofshow.models.adapter_b200 import T2IAdapter
+    if not os.path.isdir(model_dir):
+        raise FileNotFoundError(f'T2I-Adapter {model_dir!r} is not a local directory: hub ids are not downloaded; pass a '
+                                'directory holding config.json and diffusion_pytorch_model.safetensors')
+    with open(os.path.join(model_dir, 'config.json')) as f:
+        cfg = json.load(f)
+    adapter = T2IAdapter(in_channels=cfg.get('in_channels', 3), channels=cfg.get('channels', [320, 640, 1280, 1280]),
+                         num_res_blocks=cfg.get('num_res_blocks', 2), downscale_factor=cfg.get('downscale_factor', 8),
+                         adapter_type=cfg.get('adapter_type', 'full_adapter'), device=device)
+    adapter.load_state_dict(_read_weights(model_dir, ADAPTER_WEIGHTS))
+    return adapter
+
+
+def save_t2i_adapter(adapter, model_dir):
+    c = adapter.config
+    cfg = {'_class_name': 'T2IAdapter', '_diffusers_version': '0.19.3', 'adapter_type': c.adapter_type,
+           'channels': list(c.channels), 'downscale_factor': c.downscale_factor, 'in_channels': c.in_channels,
+           'num_res_blocks': c.num_res_blocks}
+    os.makedirs(model_dir, exist_ok=True)
+    with open(os.path.join(model_dir, 'config.json'), 'w') as f:
+        json.dump(cfg, f, indent=2, sort_keys=True)
+    _write_weights(model_dir, ADAPTER_WEIGHTS[0], adapter.state_dict())
 
 
 def save_combined_model(model_dir, unet, text_encoder, new_concept_cfg, tokenizer=None):

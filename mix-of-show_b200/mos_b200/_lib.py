@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(os.path.dirname(_HERE), 'lib', 'libmos_sm100.so')
 MOS_OUT_BF16, MOS_OUT_HEADS, MOS_OUT_F32 = 0, 1, 2
 MOS_DT_BF16, MOS_DT_F16 = 0, 1
 MOS_SEG_ROWS, MOS_SEG_TRANSPOSED = 0, 1
+MOS_ACT_NONE, MOS_ACT_RELU = 0, 1
 
 c_i32, c_i64, c_f32, c_vp = ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p
 
@@ -32,6 +33,7 @@ class GemmArgs(ctypes.Structure):
         ('a_dtype', c_i32), ('w_dtype', c_i32), ('pair_mode', c_i32),
         ('tile_counters', c_vp), ('tile_counters_len', c_i32),
         ('prefetch_ptr', c_vp), ('prefetch_bytes', c_i64),
+        ('act', c_i32),
     ]
 
 

@@ -7,7 +7,8 @@ import ctypes
 import torch
 
 from . import _lib
-from ._lib import MOS_OUT_BF16, MOS_OUT_F32, MOS_OUT_HEADS, GemmArgs, act_dtype, check, current_stream, ptr
+from ._lib import (MOS_ACT_NONE, MOS_ACT_RELU, MOS_OUT_BF16, MOS_OUT_F32, MOS_OUT_HEADS, GemmArgs, act_dtype, check,
+                   current_stream, ptr)
 
 BN = 160
 BK = 64
@@ -20,12 +21,13 @@ def _dt(*tensors):
 def gemm(A, W, out=None, *, bias=None, bias_batch=None, rows_per_batch=0, residual=None, geglu=False,
          lora_down=None, lora_up=None, lora_seg=0, conv=None, splits=1, partial=None, stages=0,
          out_f32=False, heads=None, M=None, lda=None, ldc=None, ldr=None, bias_batch_ld=0, accumulate=False,
-         w_static=False, pair_mode=0, counters=None, prefetch=None):
+         w_static=False, pair_mode=0, counters=None, prefetch=None, act=None):
     """out = epilogue(A @ W^T [+ LoRA]).
 
     A: bf16 / fp16 [M, K] (row pitch lda) or, with conv=(B, H, Wd, C), the NHWC activation [B, H, Wd, C]; the 16-bit
     outputs and the residual have A's dtype.  W: bf16 (weights) or fp16 (activations, Gram products) [N, K] (conv: [N, 9*C]).  heads: dict(seg_ptr=[...], seg_kind=[...], seg_rows_pad=[...], heads=,
     head_dim=, dpad=, dv_pad=, tokens_per_batch=) selects the head-split epilogue (Q/K rows, V transposed).
+    act: None or 'relu', applied to acc + bias before the residual (16-bit row output without split-K / geglu / LoRA).
     """
     a = GemmArgs()
     a.a_dtype = act_dtype(A, residual, None if out_f32 or heads is not None else out,
@@ -58,6 +60,7 @@ def gemm(A, W, out=None, *, bias=None, bias_batch=None, rows_per_batch=0, residu
     a.geglu = 1 if geglu else 0
     a.w_static = 1 if w_static else 0      # reserved (ignored by the library)
     a.pair_mode = pair_mode
+    a.act = {None: MOS_ACT_NONE, 'relu': MOS_ACT_RELU}[act]
     if prefetch is not None:               # a later launch's weights: staged in L2 by this launch (no-op semantically)
         a.prefetch_ptr, a.prefetch_bytes = ptr(prefetch), prefetch.numel() * prefetch.element_size()
     if counters is not None:               # split-K with the in-kernel finalize (zeroed int32 counters, one per output tile)
@@ -84,6 +87,25 @@ def gemm(A, W, out=None, *, bias=None, bias_batch=None, rows_per_batch=0, residu
             a.ldc = out.stride(0) if ldc is None else ldc
     check(_lib.lib().mos_gemm_bf16(ctypes.byref(a), current_stream()), 'mos_gemm_bf16')
     return out
+
+
+def pixel_unshuffle(x, y, *, r, ldy=None):
+    """PixelUnshuffle(r) of fp32 NCHW x [B, C, H, W] -> 16-bit NHWC rows y [B*(H/r)*(W/r), C*r*r] (row pitch ldy)."""
+    assert x.dtype == torch.float32 and x.is_contiguous()
+    B, C, H, W = x.shape
+    check(_lib.lib().mos_pixel_unshuffle(ptr(x), ctypes.c_int32(B), ctypes.c_int32(C), ctypes.c_int32(H), ctypes.c_int32(W),
+                                         ctypes.c_int32(r), ptr(y), ctypes.c_int64(y.stride(0) if ldy is None else ldy),
+                                         _dt(y), current_stream()), 'mos_pixel_unshuffle')
+    return y
+
+
+def avgpool2x2(x, y, *, B, H, W, C, ldx=None, ldy=None):
+    """AvgPool2d(2, 2, ceil_mode=True) over 16-bit NHWC rows: x [B*H*W, ldx] -> y [B*ceil(H/2)*ceil(W/2), ldy]."""
+    check(_lib.lib().mos_avgpool2x2(ptr(x), ctypes.c_int64(x.stride(0) if ldx is None else ldx), ctypes.c_int32(B),
+                                    ctypes.c_int32(H), ctypes.c_int32(W), ctypes.c_int32(C), ptr(y),
+                                    ctypes.c_int64(y.stride(0) if ldy is None else ldy), _dt(x, y), current_stream()),
+          'mos_avgpool2x2')
+    return y
 
 
 def splitk_finalize(partial, splits, M, N, out, *, bias=None, bias_batch=None, rows_per_batch=0, residual=None,
